@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Extract-stage throughput benchmark (BASELINE.json: audio-seconds per second at 1/2/4/8 B200; % of tensor / HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 4|3|2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 4|3|2] [--impl reference] [--dump-outputs DIR]
 
 One *step* = the whole hot path over the workload: fused log-mel front-end -> every 512-frame window through the
 hFT-Transformer -> piano-rolls stitched on the device -> device note decoding -> note records on the host.
@@ -22,6 +22,10 @@ inside the timed region) and, for N > 1, the final gather; `roofline` = the domi
 a separate profiled pass of the device leg) against the measured bf16 peak; `frontend` / `frontend_10h` = the log-mel
 kernel against the measured HBM peak; `cpu_baseline` = the oracle port (torch CPU restatement of the reference) on this
 box's host cores over a bounded sample.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned as DIR/<name>.npy (float64 or
+float32, under 64 MB in all; see `dump_notes` / `dump_features`).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -108,6 +112,41 @@ def make_wave(song_index, n_samples=SONG_SAMPLES):
     return synth.noise(n_samples, seed=1234 + song_index)
 
 
+DUMP_RECORDS = 1 << 20      # note records kept by --dump-outputs: 6 float64 columns, 48 MB at most
+DUMP_ROWS = 16384           # log-mel rows kept by --dump-outputs of config 2: 16 MB of float32
+
+
+def dump_notes(out_dir, recs, song_ids):
+    """--dump-outputs of configs 4 and 3: the note records (what extract_many(as_dicts=False) returns) of rank 0's songs.
+    note_counts.npy: the record count of each song, in the order of `song_ids`; note_{song,index,pitch,velocity,onset,
+    offset}.npy: every record when all songs together hold at most DUMP_RECORDS, else DUMP_RECORDS / len(recs) records per
+    song at sorted positions drawn by a generator seeded with the song's index.  The positions depend only on the song and
+    its record count, so two builds that compute the same notes write identical files."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = [len(r) for r in recs]
+    per_song = sum(counts) if sum(counts) <= DUMP_RECORDS else DUMP_RECORDS // len(recs)
+    cols = {k: [np.zeros(0)] for k in ("song", "index", "pitch", "velocity", "onset", "offset")}
+    for s, r in zip(song_ids, recs):
+        n = len(r)
+        idx = np.arange(n) if n <= per_song else np.sort(np.random.default_rng(s).choice(n, per_song, replace=False))
+        cols["song"].append(np.full(len(idx), s))
+        cols["index"].append(idx)
+        for k in ("pitch", "velocity", "onset", "offset"):
+            cols[k].append(r[k][idx])
+    np.save(os.path.join(out_dir, "note_counts.npy"), np.asarray(counts, np.float64))
+    for k, v in cols.items():
+        np.save(os.path.join(out_dir, f"note_{k}.npy"), np.concatenate(v).astype(np.float64))
+
+
+def dump_features(out_dir, feat):
+    """--dump-outputs of config 2: DUMP_ROWS rows of the last launch's log-mel features, at sorted positions drawn by a
+    generator seeded with 0 (logmel_rows.npy, float64), and those rows (logmel.npy, float32 [DUMP_ROWS, 256])."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(feat.shape[0], min(DUMP_ROWS, feat.shape[0]), replace=False))
+    np.save(os.path.join(out_dir, "logmel_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "logmel.npy"), feat[torch.from_numpy(rows).to(feat.device)].float().cpu().numpy())
+
+
 def cpu_baseline_sample(threads, windows=4, repeats=1):
     """Oracle port (torch fp32 CPU restatement of the reference extractor) on a bounded sample: log-mel + `windows`
     windows + note decoding of one synthetic clip.  Returns (audio-s/s, description)."""
@@ -166,7 +205,7 @@ def run_reference(args):
     print(json.dumps(line))
 
 
-def frontend_10h(ex, steps=20, warmup=3):
+def frontend_10h(ex, steps=20, warmup=3, dump_dir=None):
     """BASELINE config 2: log-mel front-end over 150 four-minute songs (10 h, 576 M samples) resident in HBM; HBM roofline with
     the algorithmic bytes of SURVEY 8(d): 4 B per sample in + 4 B x 256 per frame out (intermediates never touch HBM)."""
     from etude_b200 import synth
@@ -192,6 +231,8 @@ def frontend_10h(ex, steps=20, warmup=3):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / steps
+    if dump_dir:
+        dump_features(dump_dir, feat)
     del feat, wave
     torch.cuda.empty_cache()
     pk = peaks()
@@ -220,11 +261,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-windows", type=int, default=4)
     ap.add_argument("--frontend-microbench", action="store_true", help="same as --config 2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (seeded sample, under 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path; --impl reference has no device outputs")
     if args.frontend_microbench:
         args.config = 2
     if args.steps is None:
         args.steps = {4: 3, 3: 20, 2: 60}[args.config]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.window_batch is None:
         args.window_batch = 64 if args.config == 3 else 32
     args.warmup = max(3, args.warmup)
@@ -246,9 +293,10 @@ def main():
     from etude_b200 import AMTAPC_Extractor, ExtractorConfig, sharding
     from etude_b200.weights import default_state_dict
     sd = default_state_dict(seed=0)
-    ckpt = os.path.join(tempfile.gettempdir(), f"etude_bench_sd_{rank}.pth")
-    torch.save(sd, ckpt)
-    ex = AMTAPC_Extractor(ExtractorConfig(), ckpt, device=dev, max_windows=args.window_batch)
+    with tempfile.TemporaryDirectory() as tmp:     # the extractor reads the checkpoint in its constructor
+        ckpt = os.path.join(tmp, "sd.pth")
+        torch.save(sd, ckpt)
+        ex = AMTAPC_Extractor(ExtractorConfig(), ckpt, device=dev, max_windows=args.window_batch)
     eng = ex.engine
     pk = peaks()
 
@@ -256,7 +304,7 @@ def main():
         if rank == 0:
             sampler = ClockSampler(local)
             sampler.start()
-            fe = frontend_10h(ex, steps=args.steps, warmup=args.warmup)
+            fe = frontend_10h(ex, steps=args.steps, warmup=args.warmup, dump_dir=args.dump_outputs)
             clocks = sampler.stop()
             print(json.dumps({
                 "metric": "logmel_frontend_audio_seconds_per_second", "value": fe["audio_s_per_s"], "unit": UNIT, "n_gpus": 1, "steps": args.steps,
@@ -335,6 +383,8 @@ def main():
     ms_total = max_over_ranks(ms_total)
     launches = eng.profile_read()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_notes(args.dump_outputs, [recs] if window_sharded else recs, mine)
     ms_per_step = ms_total / args.steps
     value = audio_seconds_total / (ms_per_step / 1e3)
 
@@ -356,7 +406,7 @@ def main():
 
     step_e2e()
     barrier()
-    e2e_steps = max(5, args.steps)
+    e2e_steps = args.steps
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
         if flush is not None:

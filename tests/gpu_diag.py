@@ -5,6 +5,7 @@
 import ctypes
 import os
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -569,8 +570,10 @@ def make_extractor(max_windows=4):
     from etude_b200 import AMTAPC_Extractor, ExtractorConfig
     from oracle import model as omodel
     sd = omodel.init_state_dict(0)
-    torch.save(sd, "/tmp/etude_diag_sd.pth")
-    return AMTAPC_Extractor(ExtractorConfig(), "/tmp/etude_diag_sd.pth", device="cuda:0", max_windows=max_windows), sd
+    with tempfile.TemporaryDirectory() as tmp:     # the extractor reads the checkpoint in its constructor
+        path = os.path.join(tmp, "sd.pth")
+        torch.save(sd, path)
+        return AMTAPC_Extractor(ExtractorConfig(), path, device="cuda:0", max_windows=max_windows), sd
 
 
 def diag_logmel():

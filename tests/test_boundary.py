@@ -117,17 +117,21 @@ def test_config_mirror_matches_reference_defaults_and_rejects_other_shapes():
 
 
 def test_reference_config_object_is_accepted():
-    ref = "/root/reference"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not mounted (GPU box)")
-    import sys
-    sys.path.insert(0, ref)
-    try:
-        from etude.config import load_config
-    finally:
-        sys.path.remove(ref)
+    """The reference's `load_config().extractor` is a pydantic tree, not our dataclasses: validate() must accept any
+    object with the same attributes.  tests/golden/reference_extractor_config.json holds the values of that object
+    (etude/config/schema.py:68-131, SURVEY.md section 8), the ones the reference ran with when it made the other goldens;
+    it is read back as a plain attribute tree, and the mirror's defaults must equal it field for field."""
+    import json
+    from types import SimpleNamespace
+
     from etude_b200 import config as cfg
-    cfg.validate(load_config().extractor)
+    with open(os.path.join(ROOT, "tests", "golden", "reference_extractor_config.json")) as f:
+        ref = json.load(f, object_hook=lambda d: SimpleNamespace(**d))
+    assert cfg.validate(ref) is ref
+    mine = cfg.ExtractorConfig()
+    for section, fields in vars(ref).items():
+        for name, value in vars(fields).items():
+            assert getattr(getattr(mine, section), name) == value, f"extractor.{section}.{name}"
 
 
 def test_window_bookkeeping_matches_reference_padding():

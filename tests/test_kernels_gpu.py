@@ -377,7 +377,7 @@ def test_smoke_entry():
     g.smoke()
 
 
-def test_rolls_with_outlier_weights_vs_oracle():
+def test_rolls_with_outlier_weights_vs_oracle(tmp_path):
     """The parity goldens use default-initialised weights.  A trained checkpoint has outlier LayerNorm gains, larger FFN
     weights and more confident heads, which stress the bf16 activation stream between the kernels (ADVICE round 1).  This
     perturbs the seeded weights that way (no checkpoint can be downloaded here) and holds one window of the device path
@@ -396,7 +396,7 @@ def test_rolls_with_outlier_weights_vs_oracle():
             v *= 1.6
         elif ("fc_onset" in k or "fc_offset" in k or "fc_mpe" in k or "fc_velocity" in k) and k.endswith("weight"):
             v *= 2.0
-    path = "/tmp/etude_outlier_sd.pth"
+    path = tmp_path / "outlier_sd.pth"
     torch.save(sd, path)
     ex = AMTAPC_Extractor(ExtractorConfig(), path, device="cuda:0", max_windows=2)
     wave = synth.tones(256 * 500 + 7, 5)                     # one window
