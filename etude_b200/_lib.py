@@ -20,6 +20,13 @@ class Note(ctypes.Structure):
                 ("offset", ctypes.c_double)]
 
 
+class PcmSong(ctypes.Structure):
+    """etude_pcm_song_t"""
+    _fields_ = [("byte_offset", ctypes.c_int64), ("n_frames", ctypes.c_int64), ("frame_stride", ctypes.c_int64),
+                ("channel_stride", ctypes.c_int64), ("dst_offset", ctypes.c_int64), ("channels", ctypes.c_int32),
+                ("sample_rate", ctypes.c_int32), ("format", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 class EtudeError(RuntimeError):
     pass
 
@@ -38,6 +45,8 @@ SIGNATURES = {
                                            ctypes.c_int, c_vp]),
     "etude_resampled_length": (ctypes.c_int64, [ctypes.c_int64, ctypes.c_int, ctypes.c_int]),
     "etude_ingest": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_vp, c_vp]),
+    "etude_ingest_reserve": (ctypes.c_int, [c_vp, ctypes.POINTER(ctypes.c_int), ctypes.c_int, ctypes.c_int]),
+    "etude_ingest_pcm": (ctypes.c_int, [c_vp, c_vp, ctypes.POINTER(PcmSong), ctypes.c_int, ctypes.c_int, c_vp, c_vp]),
     "etude_forward_windows": (ctypes.c_int, [c_vp, c_vp, c_i64p, c_i64p, ctypes.c_int, ctypes.POINTER(c_vp),
                                              ctypes.POINTER(c_vp), c_vp, c_vp, c_vp, c_vp, ctypes.c_size_t, c_vp]),
     "etude_n_frame": (ctypes.c_int, [c_vp]),

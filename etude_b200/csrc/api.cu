@@ -120,8 +120,9 @@ struct LayerW {
     Linear f1, f2;    // FFN
 };
 
-enum ProfClass { PC_LOGMEL = 0, PC_EMBED, PC_GEMM_BIAS, PC_GEMM_LN, PC_GEMM_HEADS, PC_ATTN, PC_NOTES, PC_TRANSPOSE, PC_CHAIN, PC_ATTN_FUSED, PC_COUNT };
-static const char* kProfNames[PC_COUNT] = {"logmel", "embed", "gemm_bias", "gemm_ln", "gemm_heads", "attention", "notes", "transpose", "chain", "attention_fused"};
+enum ProfClass { PC_LOGMEL = 0, PC_EMBED, PC_GEMM_BIAS, PC_GEMM_LN, PC_GEMM_HEADS, PC_ATTN, PC_NOTES, PC_TRANSPOSE, PC_CHAIN, PC_ATTN_FUSED, PC_INGEST, PC_COUNT };
+static const char* kProfNames[PC_COUNT] = {"logmel", "embed", "gemm_bias", "gemm_ln", "gemm_heads", "attention", "notes", "transpose", "chain", "attention_fused",
+                                           "ingest"};
 
 // Launch accounting (always on) and optional CUDA-event timing of every launch, per kernel class.
 struct Profile {
@@ -156,7 +157,10 @@ struct etude_handle {
     int frames = kFrames;  // frames per window: 512 (AMT-APC extractor) or 128 (HFT_Transformer), from the weight count
     std::vector<void*> allocs;
     // front-end tables
-    struct ResampleTable { float* d_kern; int orig, nw, width, K; };
+    struct ResampleTable {   // polyphase kernel + the block tables of ingest_pcm_kernel (ingest.cuh)
+        float* d_kern; float4* d_btab; int* d_bstart;
+        int orig, nw, width, K, P, nb, W, sp_in, S;
+    };
     std::map<std::pair<int, int>, ResampleTable> resample_tabs;  // (sr_in, sr_out) -> polyphase kernel (etude_ingest)
     LogmelTables tab{};
     float2* tw32x32 = nullptr;  // [32 k1][32 n2] W_1024^(n2 k1) (logmel2.cuh)
@@ -537,13 +541,14 @@ static int set_func_attrs_once() {
     set_smem((const void*)chain3_kernel<true>, kChain3SmemBytes);
     set_smem((const void*)chain3_kernel<false>, kChain3SmemBytes);
     set_smem((const void*)embed2_kernel, kEmbed2SmemBytes);
-    // The note-decoding kernels run on a second stream beside the model kernels (extract_many).  An SM has ONE L1 / shared
+    set_smem((const void*)ingest_pcm_kernel, kIngestSmemBudget);
+    // The note-decoding kernels (and the ingest of extract_files) run on other streams beside the model kernels.  An SM has ONE L1 / shared
     // memory split at a time: with the default (L1-heavy) carve-out a resident notes block keeps every model CTA (which
     // needs the 227 KB split) off its SM until it finishes, and the statically partitioned model kernel waits for it.
     auto max_smem_carveout = [&](const void* fn) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
     };
-    for (const void* fn : {(const void*)notes_transpose_kernel, (const void*)notes_scan_kernel, (const void*)notes_walk_kernel,
+    for (const void* fn : {(const void*)ingest_pcm_kernel, (const void*)notes_transpose_kernel, (const void*)notes_scan_kernel, (const void*)notes_walk_kernel,
                            (const void*)notes_compact_kernel, (const void*)notes_bases_kernel, (const void*)notes_rank_kernel})
         max_smem_carveout(fn);
     set_smem((const void*)logmel2_kernel, kLogmel2SmemBytes);
@@ -907,6 +912,7 @@ extern "C" int64_t etude_resampled_length(int64_t n_in, int sr_in, int sr_out) {
 
 // torchaudio.functional._get_sinc_resample_kernel (sinc_interp_hann, lowpass_filter_width 6, rolloff 0.99): indices in
 // float64, the phase term -p / new rounded to float32 first (an int64 tensor divided by an int is float32 in torch).
+// Besides the full [new][K] table: each phase's non-zero span and the 4-output block tables of ingest_pcm_kernel.
 static int build_resample_table(etude_handle* h, int sr_in, int sr_out, etude_handle::ResampleTable* out) {
     auto it = h->resample_tabs.find({sr_in, sr_out});
     if (it != h->resample_tabs.end()) { *out = it->second; return 0; }
@@ -927,30 +933,166 @@ static int build_resample_table(etude_handle* h, int sr_in, int sr_out, etude_ha
             kern[(size_t)p * K + k] = (float)(v * window * scale);
         }
     }
-    etude_handle::ResampleTable tab{nullptr, orig, nw, width, K};
+    etude_handle::ResampleTable tab{};
+    tab.orig = orig; tab.nw = nw; tab.width = width; tab.K = K;
+    std::vector<int> lo(nw, 0), hi(nw, 0);   // non-zero span [lo, hi) of every phase
+    for (int p = 0; p < nw; ++p) {
+        const float* r = &kern[(size_t)p * K];
+        int a = 0, b = K;
+        while (a < K && r[a] == 0.f) ++a;
+        while (b > a && r[b - 1] == 0.f) --b;
+        lo[p] = a < b ? a : 0;
+        hi[p] = a < b ? b : 0;
+    }
+    // blocks of 4 consecutive outputs over a super-period of P = lcm(nw, 4) outputs: window = union of the 4 spans
+    tab.P = (int)((int64_t)nw * 4 / igcd(nw, 4));
+    tab.nb = tab.P / 4;
+    tab.sp_in = tab.P / nw * orig;
+    std::vector<int> bstart(tab.nb), bend(tab.nb);
+    for (int b = 0; b < tab.nb; ++b) {
+        int st = INT32_MAX, en = 0;
+        for (int r = 0; r < 4; ++r) {
+            const int j = 4 * b + r, p = j % nw, rel = j / nw * orig;
+            st = std::min(st, rel + lo[p]);
+            en = std::max(en, rel + hi[p]);
+        }
+        bstart[b] = st;
+        bend[b] = std::max(en, st);
+        tab.W = std::max(tab.W, bend[b] - st);
+    }
+    const int64_t tab_bytes = (int64_t)tab.nb * tab.W * 16 + (int64_t)((tab.nb + 3) & ~3) * 4;
+    auto smem = [&](int64_t S) { return tab_bytes + 4 * (S * tab.sp_in - orig + K + tab.W); };
+    tab.S = smem(32) <= kIngestSmemBudget ? 32 : 0;     // unstaged when 32 super-periods do not fit
+    while (tab.S && (int64_t)tab.S * tab.nb < 1024 && smem(2 * tab.S) <= 80 * 1024) tab.S *= 2;   // >= 4 blocks per thread
+    if (tab.S) {
+        std::vector<float4> bt((size_t)tab.nb * tab.W, make_float4(0.f, 0.f, 0.f, 0.f));
+        for (int b = 0; b < tab.nb; ++b)
+            for (int r = 0; r < 4; ++r) {
+                const int j = 4 * b + r, p = j % nw, rel = j / nw * orig;
+                for (int k = lo[p]; k < hi[p]; ++k) (&bt[(size_t)b * tab.W + rel + k - bstart[b]].x)[r] = kern[(size_t)p * K + k];
+            }
+        if (dev_upload(h, &tab.d_btab, bt.data(), bt.size()) || dev_upload(h, &tab.d_bstart, bstart.data(), bstart.size())) return -1;
+    }
     if (dev_upload(h, &tab.d_kern, kern.data(), kern.size())) return -1;
     h->resample_tabs[{sr_in, sr_out}] = tab;
     *out = tab;
     return 0;
 }
 
+extern "C" int etude_ingest_reserve(etude_handle_t* h, const int* sample_rates, int n, int sr_out) {
+    if (!h || (n > 0 && !sample_rates) || n < 0 || sr_out <= 0) return fail("etude_ingest_reserve: bad argument");
+    CUDA_OK(cudaSetDevice(h->device));
+    for (int i = 0; i < n; ++i) {
+        if (sample_rates[i] <= 0) return fail("etude_ingest_reserve: sample rate %d", sample_rates[i]);
+        etude_handle::ResampleTable tab;
+        if (sample_rates[i] != sr_out && build_resample_table(h, sample_rates[i], sr_out, &tab)) return -1;
+    }
+    return 0;
+}
+
+static int pcm_container_bytes(int fmt) {
+    switch (fmt) {
+        case ETUDE_PCM_U8: return 1;
+        case ETUDE_PCM_S16: return 2;
+        case ETUDE_PCM_S24: return 3;
+        case ETUDE_PCM_S32: case ETUDE_PCM_F32: return 4;
+        case ETUDE_PCM_F64: return 8;
+        default: return 0;
+    }
+}
+
+extern "C" int etude_ingest_pcm(etude_handle_t* h, const void* pcm_dev, const etude_pcm_song_t* songs, int n_songs, int sr_out,
+                                float* wave_out_dev, void* stream) {
+    if (!h || !pcm_dev || !songs || !wave_out_dev) return fail("etude_ingest_pcm: null argument");
+    if (n_songs < 1 || sr_out <= 0) return fail("etude_ingest_pcm: n_songs=%d, sr_out=%d", n_songs, sr_out);
+    static_assert(ETUDE_PCM_U8 == PCM_U8 && ETUDE_PCM_S16 == PCM_S16 && ETUDE_PCM_S24 == PCM_S24 && ETUDE_PCM_S32 == PCM_S32 &&
+                  ETUDE_PCM_F32 == PCM_F32 && ETUDE_PCM_F64 == PCM_F64, "format codes");
+    CUDA_OK(cudaSetDevice(h->device));
+    std::vector<PcmSongDev> dev(n_songs);
+    std::vector<double> flops(n_songs), bytes(n_songs);
+    for (int i = 0; i < n_songs; ++i) {   // everything is checked before the first launch
+        const etude_pcm_song_t& s = songs[i];
+        const int cb = pcm_container_bytes(s.format);
+        if (!cb) return fail("etude_ingest_pcm: song %d: unknown format %d", i, s.format);
+        if (s.channels < 1 || s.channels > 64) return fail("etude_ingest_pcm: song %d: %d channels (1..64)", i, s.channels);
+        if (s.n_frames < 1 || s.sample_rate <= 0) return fail("etude_ingest_pcm: song %d: %lld frames at %d Hz", i, (long long)s.n_frames, s.sample_rate);
+        if (s.byte_offset < 0 || s.dst_offset < 0 || s.frame_stride < cb || (s.channels > 1 && s.channel_stride < cb))
+            return fail("etude_ingest_pcm: song %d: bad offsets or strides (offset %lld, frame stride %lld, channel stride %lld, dst %lld)", i,
+                        (long long)s.byte_offset, (long long)s.frame_stride, (long long)s.channel_stride, (long long)s.dst_offset);
+        const int al = cb == 3 ? 1 : cb;
+        if (((uintptr_t)pcm_dev + s.byte_offset) % al || s.frame_stride % al || s.channel_stride % al)
+            return fail("etude_ingest_pcm: song %d: offset / strides not aligned to its %d-byte samples", i, cb);
+        PcmSongDev& d = dev[i];
+        d = PcmSongDev{};
+        d.src = (const uint8_t*)pcm_dev + s.byte_offset;
+        d.out = wave_out_dev + s.dst_offset;
+        d.n_frames = s.n_frames;
+        d.n_out = etude_resampled_length(s.n_frames, s.sample_rate, sr_out);
+        d.frame_stride = s.frame_stride;
+        d.chan_stride = s.channels > 1 ? s.channel_stride : 0;
+        d.fmt = s.format;
+        d.channels = s.channels;
+        if (d.n_out < 1) return fail("etude_ingest_pcm: song %d: empty output", i);
+        int64_t taps = 0;
+        if (s.sample_rate != sr_out) {
+            etude_handle::ResampleTable tab;
+            if (build_resample_table(h, s.sample_rate, sr_out, &tab)) return -1;
+            d.kern = tab.d_kern; d.btab = tab.d_btab; d.bstart = tab.d_bstart;
+            d.orig = tab.orig; d.nw = tab.nw; d.width = tab.width; d.K = tab.K;
+            d.P = tab.P; d.nb = tab.nb; d.W = tab.W; d.sp_in = tab.sp_in; d.S = tab.S;
+            taps = tab.S ? (int64_t)tab.W : (int64_t)tab.K;   // per output, as visited
+        }
+        if (d.kern && d.S) {
+            const int64_t n_sp = (d.n_out + d.P - 1) / d.P;
+            d.n_tiles = (int)((n_sp + d.S - 1) / d.S);
+        } else {
+            d.n_tiles = (int)((d.n_out + kIngestFlatTile - 1) / kIngestFlatTile);
+        }
+        flops[i] = 2.0 * (double)taps * (double)d.n_out;
+        bytes[i] = (double)s.n_frames * s.channels * cb + 4.0 * (double)d.n_out;
+    }
+    if (set_func_attrs_once()) return -1;
+    cudaStream_t st = (cudaStream_t)stream;
+    int per_sm = 0;
+    for (int a = 0; a < n_songs; a += kIngestMaxSongs) {
+        IngestLaunch L{};
+        L.n_songs = std::min(kIngestMaxSongs, n_songs - a);
+        int tiles = 0;
+        size_t smem = 0;
+        double fl = 0, by = 0;
+        for (int i = 0; i < L.n_songs; ++i) {
+            PcmSongDev& d = dev[a + i];
+            d.tile0 = tiles;
+            tiles += d.n_tiles;
+            if (d.kern && d.S)
+                smem = std::max(smem, (size_t)d.nb * d.W * 16 + (size_t)((d.nb + 3) & ~3) * 4 + 4 * (size_t)(d.S * d.sp_in - d.orig + d.K + d.W));
+            fl += flops[a + i];
+            by += bytes[a + i];
+            L.song[i] = d;
+        }
+        CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ingest_pcm_kernel, kIngestThreads, smem));
+        const int grid = std::max(1, std::min(tiles, h->num_sms * std::max(per_sm, 1)));
+        cudaEvent_t ev = h->prof.begin(PC_INGEST, st, fl, by);
+        ingest_pcm_kernel<<<grid, kIngestThreads, smem, st>>>(L);
+        h->prof.end(ev, st);
+        CUDA_OK(cudaGetLastError());
+    }
+    return 0;
+}
+
+// One planar fp32 song through ingest_pcm_kernel.
 extern "C" int etude_ingest(etude_handle_t* h, const float* pcm, int channels, int64_t n_in, int sr_in, int sr_out, float* wave_out,
                             void* stream) {
     if (!h || !pcm || !wave_out) return fail("etude_ingest: null argument");
     if (channels < 1 || channels > 64 || n_in < 1 || sr_in <= 0 || sr_out <= 0) return fail("etude_ingest: bad shape (channels=%d, n=%lld, %d -> %d Hz)", channels, (long long)n_in, sr_in, sr_out);
-    CUDA_OK(cudaSetDevice(h->device));
-    IngestParams p{};
-    p.pcm = pcm; p.out = wave_out; p.n_in = n_in; p.channels = channels;
-    p.n_out = etude_resampled_length(n_in, sr_in, sr_out);
-    if (sr_in != sr_out) {
-        etude_handle::ResampleTable tab;
-        if (build_resample_table(h, sr_in, sr_out, &tab)) return -1;
-        p.kern = tab.d_kern; p.orig = tab.orig; p.nw = tab.nw; p.width = tab.width; p.K = tab.K;
-    }
-    if (p.n_out < 1) return fail("etude_ingest: empty output");
-    ingest_kernel<<<(unsigned)((p.n_out + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p);
-    CUDA_OK(cudaGetLastError());
-    return 0;
+    etude_pcm_song_t s{};
+    s.n_frames = n_in;
+    s.frame_stride = 4;
+    s.channel_stride = 4 * n_in;
+    s.channels = channels;
+    s.sample_rate = sr_in;
+    s.format = ETUDE_PCM_F32;
+    return etude_ingest_pcm(h, pcm, &s, 1, sr_out, wave_out, stream);
 }
 
 extern "C" int64_t etude_feature_rows(int64_t n_samples) {

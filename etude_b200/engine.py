@@ -103,6 +103,33 @@ class Engine:
             _lib.check(self.lib.etude_ingest(self._h, _ptr(x), c, n, int(sr_in), int(sr_out), _ptr(out), self._stream()), "etude_ingest")
         return out
 
+    def ingest_reserve(self, sample_rates, sr_out=16000):
+        """Builds the resampling tables of these input rates now (a synchronous upload each), not inside a pipeline."""
+        rates = sorted({int(r) for r in sample_rates})
+        with torch.cuda.device(self.index):
+            _lib.check(self.lib.etude_ingest_reserve(self._h, (ctypes.c_int * max(1, len(rates)))(*rates), len(rates), int(sr_out)),
+                       "etude_ingest_reserve")
+
+    def ingest_pcm(self, raw_dev, infos, sr_out=16000):
+        """Raw PCM of many WAV files (audio.WavInfo) in one launch: ``raw_dev`` is a uint8 CUDA tensor holding their data
+        chunks at audio.raw_layout(infos).  Returns (wave_dev, wave_off, n_samples): the songs' mono ``sr_out`` waves back
+        to back in one fp32 tensor, as ``ingest`` returns them for the same samples converted to float."""
+        from .audio import raw_layout
+        offs, total = raw_layout(infos)
+        if not (raw_dev.is_cuda and raw_dev.dtype == torch.uint8 and raw_dev.numel() >= total):
+            raise ValueError(f"raw_dev must be a uint8 CUDA tensor of at least {total} bytes")
+        n_samples = [int(self.lib.etude_resampled_length(i.n_frames, int(i.sample_rate), int(sr_out))) for i in infos]
+        wave_off = np.concatenate([[0], np.cumsum(n_samples)]).astype(np.int64)
+        songs = (_lib.PcmSong * len(infos))()
+        for s, (info, o) in enumerate(zip(infos, offs)):
+            songs[s] = _lib.PcmSong(o, info.n_frames, info.frame_bytes, info.bytes_per_sample, int(wave_off[s]), info.channels,
+                                    info.sample_rate, info.format, 0)
+        out = torch.empty(max(1, int(wave_off[-1])), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.index):
+            _lib.check(self.lib.etude_ingest_pcm(self._h, _ptr(raw_dev), songs, len(infos), int(sr_out), _ptr(out), self._stream()),
+                       "etude_ingest_pcm")
+        return out, wave_off[:-1], n_samples
+
     def logmel(self, wave_dev, wave_off, n_samples):
         """wave_dev: 1-D fp32 CUDA tensor holding the songs back to back.  Returns (feat [rows,256], feat_row_off)."""
         rows = [feature_rows(n) for n in n_samples]

@@ -8,6 +8,7 @@ arithmetic done by the sm_100a kernels of libetude_b200.so.
         ._mpe2note(a_onset, a_offset, a_mpe, a_velocity, ...)      256-418
         ._note2midi / ._note2json                                  421-446
     + extract_many(waves)   additive batch API (the reference is one song, batch 1)
+    + extract_files(paths)  the same pipeline from WAV files (raw PCM converted and resampled on the device)
 
 Differences from the reference, all deliberate: CUDA only (no cpu/mps path, no fallback); default ExtractorConfig
 shapes only; windows are processed in batches and rolls stay on the device between the stages.
@@ -19,6 +20,7 @@ from typing import Optional, Union
 import numpy as np
 import torch
 
+from . import audio as _audio
 from . import config as _config
 from . import engine as _engine
 from .model import Decoder_SPEC2MIDI as Decoder
@@ -99,12 +101,11 @@ class AMTAPC_Extractor:
             self._note2midi(notes, output_midi_path, min_duration)
 
     def _wav2feature(self, audio_path: str, _on_device: bool = False) -> torch.Tensor:
-        """wav -> log-mel [T, 256].  File decoding stays on torchaudio (extractor.py:180); the channel mean and the
+        """wav -> log-mel [T, 256].  File decoding stays on torchaudio (extractor.py:180), except for WAV files where
+        torchaudio cannot decode (no TorchCodec): those are read natively (audio.load_resampled).  The channel mean and the
         Resample(sr, 16000) of extractor.py:181-184 run in the CUDA ingest kernel, the MelSpectrogram + log (186-197) in
         the fused CUDA front-end."""
-        import torchaudio
-        wave, sr = torchaudio.load(audio_path)
-        wave_mono = self.engine.ingest(wave, int(sr), int(self.config.feature.sr))
+        wave_mono = _audio.load_resampled(self.engine, audio_path, int(self.config.feature.sr))
         feat = self.wave_to_feature(wave_mono)
         return feat if _on_device else feat.cpu()
 
@@ -214,15 +215,90 @@ class AMTAPC_Extractor:
             if pinned is None or pinned.numel() < total:
                 pinned = torch.empty(total, dtype=torch.float32, pin_memory=True)
             hv = pinned.numpy()
+
+        def stage(a, b, copy_s, main):   # host staging + H2D of songs [a, b) on the copy stream
+            lo, hi = int(wave_off[a]), int(wave_off[b])
+            if wave_dev is not None:   # already resident: a view, ready as soon as the caller's stream is
+                ev = torch.cuda.Event()
+                ev.record(main)
+                return wave_dev[lo:hi], ev
+            for w, o, n in zip(waves[a:b], wave_off[a:b], n_samples[a:b]):
+                hv[o : o + n] = np.asarray(w, dtype=np.float32).reshape(-1)
+            with torch.cuda.stream(copy_s):
+                dev = pinned[lo:hi].to(self.device, non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(copy_s)
+            return dev, ev
+
+        return self._pipeline(n_samples, stage, as_dicts, return_rolls, group_songs, notes_batch)
+
+    def extract_files(self, audio_paths, output_json_paths=None, as_dicts=True, group_songs=4, notes_batch=12):
+        """The bulk form of ``extract(path, json)``: WAV files -> notes through the ``extract_many`` pipeline.
+
+        Every header is parsed first (audio.read_wav_info), so a file that is not a supported WAV or is too short (16 kHz
+        length <= 1024 samples) raises ValueError before any device work.  The staging step of a group reads its files'
+        data chunks into pinned memory, uploads the raw bytes and converts + resamples them on the device
+        (Engine.ingest_pcm), all on the copy stream while the model runs the previous group.  Pinned memory is two groups
+        of raw bytes, each buffer reused only after its upload has completed.
+
+        Returns what ``extract_many`` returns.  With ``output_json_paths`` every file's notes are also written exactly as
+        ``extract`` writes them (``min_duration`` filter, indent 2)."""
+        paths = [str(p) for p in audio_paths]
+        if output_json_paths is not None and len(output_json_paths) != len(paths):
+            raise ValueError(f"{len(paths)} audio files but {len(output_json_paths)} JSON paths")
+        if not paths:
+            return []
+        sr_out = int(self.config.feature.sr)
+        infos = [_audio.read_wav_info(p) for p in paths]
+        n_samples = [int(self.engine.lib.etude_resampled_length(i.n_frames, i.sample_rate, sr_out)) for i in infos]
+        for info, n in zip(infos, n_samples):
+            if n <= 1024:
+                raise ValueError(f"{info.path}: {info.n_frames} frames at {info.sample_rate} Hz are {n} samples at {sr_out} Hz; "
+                                 "the log-mel needs more than 1024")
+        self.engine.ingest_reserve([i.sample_rate for i in infos if i.sample_rate != sr_out], sr_out)
+        groups = _pipeline_groups(len(paths), int(group_songs)) if group_songs and group_songs > 0 else [(0, len(paths))]
+        cap = max(_audio.raw_layout(infos[a:b])[1] for a, b in groups)
+        bufs = [torch.empty(max(1, cap), dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        buf_ev = [None, None]   # H2D of each pinned buffer's last group
+        turn = [0]
+
+        def stage(a, b, copy_s, main):
+            k = turn[0] % 2
+            turn[0] += 1
+            if buf_ev[k] is not None:
+                buf_ev[k].synchronize()
+            offs, nbytes = _audio.raw_layout(infos[a:b])
+            host = bufs[k].numpy()
+            for info, o in zip(infos[a:b], offs):
+                _audio.read_wav_data(info, host[o : o + info.data_bytes])
+            with torch.cuda.stream(copy_s):
+                raw = bufs[k][:nbytes].to(self.device, non_blocking=True)
+                buf_ev[k] = torch.cuda.Event()
+                buf_ev[k].record(copy_s)
+                dev, _, _ = self.engine.ingest_pcm(raw, infos[a:b], sr_out)
+                ev = torch.cuda.Event()
+                ev.record(copy_s)
+            return dev, ev
+
+        recs = self._pipeline(n_samples, stage, False, False, group_songs, notes_batch)
+        dicts = [_engine.notes_to_dicts(r) for r in recs] if as_dicts or output_json_paths is not None else None
+        for notes, path in zip(dicts or [], output_json_paths or []):
+            self._note2json(notes, path, self.config.infer.min_duration)
+        return dicts if as_dicts else recs
+
+    def _pipeline(self, n_samples, stage, as_dicts, return_rolls, group_songs, notes_batch):
+        """The extract_many pipeline from the 16 kHz waves on; ``stage(a, b, copy_s, main)`` puts songs [a, b) back to back
+        on the device and returns (tensor, event after which it is complete)."""
         cfg = self.config.infer
         hop_sec = float(self.config.feature.hop_sample / self.config.feature.sr)
-        n_songs = len(waves)
+        n_songs = len(n_samples)
         if return_rolls or group_songs is None or group_songs <= 0:
             groups = [(0, n_songs)]
         else:
             groups = _pipeline_groups(n_songs, int(group_songs))
         if notes_batch is None or notes_batch <= 0:
             notes_batch = n_songs
+        wave_off = np.concatenate([[0], np.cumsum(n_samples)]).astype(np.int64)
         song_rows = [_engine.feature_rows(n) - 2 * MARGIN for n in n_samples]          # T_pad per song
         song_row_off = np.concatenate([[0], np.cumsum(song_rows)]).astype(np.int64)
         rolls = self.engine.alloc_rolls(int(song_row_off[-1]), self.device)            # one set of rolls for the whole call (caller's stream)
@@ -242,20 +318,6 @@ class AMTAPC_Extractor:
         copy_s.wait_stream(main)
         notes_s.wait_stream(main)
 
-        def stage(a, b):   # host staging + H2D of songs [a, b) on the copy stream
-            lo, hi = int(wave_off[a]), int(wave_off[b])
-            if wave_dev is not None:   # already resident: a view, ready as soon as the caller's stream is
-                ev = torch.cuda.Event()
-                ev.record(main)
-                return wave_dev[lo:hi], ev
-            for w, o, n in zip(waves[a:b], wave_off[a:b], n_samples[a:b]):
-                hv[o : o + n] = np.asarray(w, dtype=np.float32).reshape(-1)
-            with torch.cuda.stream(copy_s):
-                dev = pinned[lo:hi].to(self.device, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(copy_s)
-            return dev, ev
-
         def decode(a, b, ev):  # note decoding + D2H of songs [a, b) on the notes stream, once their rolls are complete
             notes_s.wait_event(ev)
             with torch.cuda.stream(notes_s):
@@ -265,7 +327,7 @@ class AMTAPC_Extractor:
 
         recs, keep = [], []
         decoded, ready, ev_ready = 0, 0, None     # songs [decoded, ready) have complete rolls once ev_ready fires
-        staged = stage(*groups[0])
+        staged = stage(*groups[0], copy_s, main)
         for gi, (a, b) in enumerate(groups):
             dev, ev_up = staged
             main.wait_event(ev_up)
@@ -276,7 +338,7 @@ class AMTAPC_Extractor:
             ev_done.record(main)
             keep.append(dev)                # device buffers stay alive until every stream is done with them
             if gi + 1 < len(groups):
-                staged = stage(*groups[gi + 1])
+                staged = stage(*groups[gi + 1], copy_s, main)
             if ready - decoded >= notes_batch:   # decode behind the model group just enqueued
                 recs.extend(decode(decoded, ready, ev_ready))
                 decoded = ready

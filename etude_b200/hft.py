@@ -26,6 +26,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
+from . import audio as _audio
 from . import engine as _engine
 from .config import ExtractorMidiConfig
 from .weights import layout, pack_state_dict
@@ -168,10 +169,9 @@ class HFT_Transformer:
             json.dump(notes, f, ensure_ascii=False, indent=4)
 
     def _wav2feature(self, f_wav, _on_device: bool = False) -> torch.Tensor:
-        """Reference: hft_transformer.py:119-138.  wav -> log-mel [T, 256] with ``pad_mode`` from the config ("constant")."""
-        import torchaudio
-        wave, sr = torchaudio.load(f_wav)
-        wave_mono = self.engine.ingest(wave, int(sr), int(self.config.feature.sr))
+        """Reference: hft_transformer.py:119-138.  wav -> log-mel [T, 256] with ``pad_mode`` from the config ("constant").
+        WAV files torchaudio cannot decode (no TorchCodec) are read natively (audio.load_resampled)."""
+        wave_mono = _audio.load_resampled(self.engine, f_wav, int(self.config.feature.sr))
         feat = self.wave_to_feature(wave_mono)
         return feat if _on_device else feat.cpu()
 

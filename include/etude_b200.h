@@ -72,6 +72,43 @@ int64_t etude_resampled_length(int64_t n_in, int sr_in, int sr_out);
 int etude_ingest(etude_handle_t* h, const float* pcm_dev, int channels, int64_t n_in, int sr_in, int sr_out, float* wave_out_dev,
                  void* stream);
 
+/* Raw PCM sample formats of etude_ingest_pcm, converted to float32 as FFmpeg does: u8 (x - 128) / 2^7, s16 x / 2^15,
+ * s24 (3 bytes, little-endian) x / 2^23, s32 (float)x / 2^31, f32 as is, f64 rounded to f32. */
+#define ETUDE_PCM_U8 1
+#define ETUDE_PCM_S16 2
+#define ETUDE_PCM_S24 3
+#define ETUDE_PCM_S32 4
+#define ETUDE_PCM_F32 5
+#define ETUDE_PCM_F64 6
+
+/* One song of etude_ingest_pcm.  Sample (frame f, channel c) is at pcm_dev + byte_offset + f * frame_stride +
+ * c * channel_stride: interleaved frames (a WAV data chunk) have frame_stride = channels * bytes and channel_stride = bytes,
+ * planar audio has frame_stride = bytes and channel_stride = n_frames * bytes.  Offsets and strides of 2/4/8-byte samples
+ * are multiples of the sample size. */
+typedef struct {
+    int64_t byte_offset;
+    int64_t n_frames;
+    int64_t frame_stride;
+    int64_t channel_stride;
+    int64_t dst_offset;     /* first output sample in wave_out_dev */
+    int32_t channels;       /* 1..64 */
+    int32_t sample_rate;
+    int32_t format;         /* ETUDE_PCM_* */
+    int32_t reserved;
+} etude_pcm_song_t;
+
+/* Builds the resampling tables for these input rates (a synchronous upload per new rate), so that later
+ * etude_ingest_pcm / etude_ingest calls at those rates enqueue kernels only. */
+int etude_ingest_reserve(etude_handle_t* h, const int* sample_rates, int n, int sr_out);
+
+/* etude_ingest for n_songs songs of raw PCM in one device buffer, each with its own format, channel count, rate and
+ * layout (songs_host is read on the host).  Song s writes etude_resampled_length(n_frames, sample_rate, sr_out) samples at
+ * wave_out_dev + dst_offset, bit-identical to etude_ingest on the same samples converted to planar fp32.  Uses no device
+ * buffer of the handle, so it may run on another stream beside the log-mel, model and note calls.  Every song is checked
+ * before anything is launched. */
+int etude_ingest_pcm(etude_handle_t* h, const void* pcm_dev, const etude_pcm_song_t* songs_host, int n_songs, int sr_out,
+                     float* wave_out_dev, void* stream);
+
 /* Rows of the padded feature block of a song with n_samples samples: 32 + T_pad + 32 where
  * T = 1 + n_samples/256 and T_pad = ceil(T/512)*512 (extractor.py:210-213). */
 int64_t etude_feature_rows(int64_t n_samples);
