@@ -75,6 +75,9 @@ SIGNATURES = {
     "etude_k_chain": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int64, c_vp,
                                      ctypes.c_int, c_vp]),
     "etude_k_embed": (ctypes.c_int, [c_vp, c_vp, c_i64p, ctypes.c_int, c_vp, ctypes.c_int, c_vp]),
+    "etude_k_heads": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int, c_i64p, ctypes.c_int, ctypes.c_int,
+                                     ctypes.POINTER(c_vp), c_vp, c_vp]),
+    "etude_k_transpose_time": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_vp, c_vp]),
     "etude_k_attention": (ctypes.c_int, [c_vp, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_vp, ctypes.c_int,
                                          ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_vp, c_vp,
                                          c_vp]),

@@ -1217,6 +1217,45 @@ extern "C" int etude_k_embed(etude_handle_t* h, const float* feat, const int64_t
     return launch_embed(h, feat, nw, (__nv_bfloat16*)out_bf16, st, nullptr, variant >= 16 ? variant - 16 : 0);
 }
 
+static int check_rolls(const char* who, void* const rolls[4], const char* name) {
+    if (rolls)
+        for (int i = 0; i < 4; ++i)
+            if (!rolls[i]) return fail("%s: %s[%d] is null (pass %s = NULL to skip those heads)", who, name, i, name);
+    return 0;
+}
+
+// The heads GEMM of forward_impl alone, on caller-supplied weights (the epilogue is the only place the rolls are written).
+extern "C" int etude_k_heads(etude_handle_t* h, const void* x_bf16, const void* w_bf16, const float* bias, int nw, int time_major,
+                             const int64_t* out_row, int keep0, int keepn, void* const rolls[4], float* vel_logits, void* stream) {
+    if (!h || !x_bf16 || !w_bf16 || !bias || !out_row || !rolls) return fail("etude_k_heads: null argument");
+    if (check_rolls("etude_k_heads", rolls, "rolls")) return -1;
+    if (nw < 1 || nw > max_windows_of(h)) return fail("etude_k_heads: n_windows=%d out of range (1..%d)", nw, max_windows_of(h));
+    if (keep0 < 0 || keepn < 1 || keep0 + keepn > h->frames)
+        return fail("etude_k_heads: kept frames [%d, %d) outside the %d-frame window", keep0, keep0 + keepn, h->frames);
+    if (set_func_attrs_once()) return -1;
+    CUDA_OK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_OK(cudaMemcpyAsync(h->d_out_row, out_row, sizeof(int64_t) * nw, cudaMemcpyHostToDevice, st));
+    GemmParams p{};
+    p.M = nw * h->frames * kNotes; p.N = 144; p.K = 256; p.bias = bias; p.heads_time_major = time_major ? 1 : 0; p.heads_row0 = h->d_out_row;
+    p.roll_onset = (float*)rolls[0]; p.roll_offset = (float*)rolls[1]; p.roll_mpe = (float*)rolls[2];
+    p.roll_velocity = (int8_t*)rolls[3]; p.vel_logits = vel_logits;
+    p.frames = h->frames; p.keep0 = keep0; p.keepn = keepn;
+    return launch_gemm<144, EPI_HEADS>(x_bf16, w_bf16, p, GemmIO{}, st, nullptr);
+}
+
+// The decoder's time-axis transpose of forward_impl alone, with the handle's pos_time table and window length.
+extern "C" int etude_k_transpose_time(etude_handle_t* h, const void* in_bf16, int nw, void* out_bf16, void* stream) {
+    if (!h || !in_bf16 || !out_bf16) return fail("etude_k_transpose_time: null argument");
+    if (nw < 1 || nw > max_windows_of(h)) return fail("etude_k_transpose_time: n_windows=%d out of range (1..%d)", nw, max_windows_of(h));
+    CUDA_OK(cudaSetDevice(h->device));
+    const int ND = nw * h->frames * kNotes;
+    transpose_time_kernel<<<(ND + 7) / 8, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)in_bf16, h->pos_time, 16.f, ND, h->frames,
+                                                                         (__nv_bfloat16*)out_bf16);
+    CUDA_OK(cudaGetLastError());
+    return debug_sync("transpose_time", (cudaStream_t)stream);
+}
+
 // What one pass over nw windows reads and writes; the public entry points below are thin views of it.
 struct ForwardIO {
     const float* feat = nullptr;        // padded feature blocks (encoder input) ...
@@ -1302,13 +1341,6 @@ static int forward_impl(etude_handle_t* h, const ForwardIO& io, int nw, void* wo
     for (int l = 0; l < 3; ++l)
         if (self_layer(h->tim[l], ws.t, ws.dqkv, ws.dctx, nw * kNotes, F, st, prof)) return -1;
     return heads(h->heads_t, ws.t, io.rolls_B, io.vel_logits_B, 1);
-}
-
-static int check_rolls(const char* who, void* const rolls[4], const char* name) {
-    if (rolls)
-        for (int i = 0; i < 4; ++i)
-            if (!rolls[i]) return fail("%s: %s[%d] is null (pass %s = NULL to skip those heads)", who, name, i, name);
-    return 0;
 }
 
 extern "C" int etude_forward_windows(etude_handle_t* h, const float* feat, const int64_t* win_row, const int64_t* out_row, int nw,

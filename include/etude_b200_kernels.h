@@ -54,6 +54,19 @@ int etude_k_chain(const void* ctx_bf16_dev, const void* wo_bf16_dev, const float
 int etude_k_embed(etude_handle_t* h, const float* feat_dev, const int64_t* win_row_host, int n_windows, void* out_bf16_dev, int variant,
                   void* stream);
 
+/* Output heads of the decoder (reference amt_apc.py:186-189 / 217-220, extractor.py:239-248) on a handle's window length F:
+ * logits = x W^T + bias over rows of x bf16 [n_windows * F * 88, 256]; W bf16 [144, 256] (onset, offset, mpe, velocity[128],
+ * padding), bias fp32 [144].  Rows are (window, frame, note) with time_major == 0, (window, note, frame) with time_major == 1.
+ * Only window frames f in [keep0, keep0 + keepn) are written, at roll row out_row_host[w] + f - keep0 (fp32 rolls[0..2] get the
+ * three sigmoids, int8 rolls[3] the velocity argmax, first maximum on ties); no other roll row is touched.
+ * vel_logits_dev (optional): fp32 [n_windows * F * 88, 128] in (window, frame, note) order, every frame. */
+int etude_k_heads(etude_handle_t* h, const void* x_bf16_dev, const void* w_bf16_dev, const float* bias_dev, int n_windows, int time_major,
+                  const int64_t* out_row_host, int keep0, int keepn, void* const rolls_dev[4], float* vel_logits_dev, void* stream);
+
+/* Time-axis transpose of the decoder (reference amt_apc.py:203-205) on a handle's window length F:
+ * out[(w * 88 + n) * F + f, :] = bf16(16 * in[(w * F + f) * 88 + n, :] + pos_embedding_time[f, :]), bf16 [n_windows * F * 88, 256]. */
+int etude_k_transpose_time(etude_handle_t* h, const void* in_bf16_dev, int n_windows, void* out_bf16_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
