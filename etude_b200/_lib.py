@@ -72,6 +72,7 @@ SIGNATURES = {
     "etude_k_gemm": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_vp, c_vp,
                                     ctypes.c_int, c_vp, c_vp, c_vp, c_vp]),
     "etude_k_attn_qkv": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int, c_vp, c_vp]),
+    "etude_k_cross_attn": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_vp, c_vp]),
     "etude_k_chain": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int64, c_vp,
                                      ctypes.c_int, c_vp]),
     "etude_k_embed": (ctypes.c_int, [c_vp, c_vp, c_i64p, ctypes.c_int, c_vp, ctypes.c_int, c_vp]),

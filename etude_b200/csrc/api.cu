@@ -16,6 +16,7 @@
 #include "attn_qkv.cuh"
 #include "attn_pair.cuh"
 #include "chain3.cuh"
+#include "cross_attn.cuh"
 #include "embed2.cuh"
 #include "gemm.cuh"
 #include "logmel.cuh"
@@ -171,7 +172,8 @@ struct etude_handle {
     __nv_bfloat16* w_embed_bf16 = nullptr;  // [256][64] taps 0..63 of W16 (embed2.cuh)
     float* w64 = nullptr;                   // [256] tap 64
     LayerW enc[3], dec0, dec[2], tim[3];
-    Linear kv_all;  // the three cross-attention K|V projections [1536,256]
+    Linear kv_hm;   // the three cross-attention K|V projections, head-major: row 512 l + 128 h + {0..63 Wk_h, 64..127 Wv_h}
+    Linear kv2;     // layer 2's K|V [512,256] (K then V): only the attention-probabilities output (attention2) reads it
     __nv_bfloat16* q0 = nullptr;  // fc_q(pos_embedding_freq) of layer zero, [128,256] (rows >= 88 zero)
     float* pos_freq = nullptr;    // decoder.pos_embedding_freq [88,256] (+ wrap rows)
     __nv_bfloat16* pos_freq_bf16 = nullptr;  // the same table, bf16, three times over [264,256]: chain residual, row % 88
@@ -401,11 +403,22 @@ extern "C" int etude_create(int device, const float* weights_host, size_t n_floa
         RawLinear f2 = take_linear(bl, 256, 512);
         return upload_raw(h, &L.f1, f1, 512, 256) || upload_raw(h, &L.f2, f2, 256, 512);
     };
-    std::vector<float> kvw, kvb;  // cross-attention K|V of the three decoder layers
+    std::vector<float> kvw((size_t)1536 * 256), kvb(1536), kv2w, kv2b;  // cross-attention K|V of the three decoder layers
+    int n_cross = 0;
     auto take_cross = [&](LayerW& L, RawMha* keep) -> int {
         RawMha m = take_mha(bl);
-        append(kvw, m.k.w, 65536); append(kvw, m.v.w, 65536);
-        append(kvb, m.k.b, 256); append(kvb, m.v.b, 256);
+        const int l = n_cross++;
+        for (int hd = 0; hd < 4; ++hd)   // head-major for cross_attn.cuh: [Wk_h; Wv_h] of head h at rows 512 l + 128 h
+            for (int part = 0; part < 2; ++part) {
+                const RawLinear& src = part ? m.v : m.k;
+                const size_t row = (size_t)l * 512 + hd * 128 + part * 64;
+                memcpy(&kvw[row * 256], src.w + (size_t)hd * 64 * 256, (size_t)64 * 256 * sizeof(float));
+                memcpy(&kvb[row], src.b + hd * 64, 64 * sizeof(float));
+            }
+        if (l == 2) {
+            append(kv2w, m.k.w, 65536); append(kv2w, m.v.w, 65536);
+            append(kv2b, m.k.b, 256); append(kv2b, m.v.b, 256);
+        }
         if (keep) *keep = m;
         return upload_raw(h, &L.cq, m.q, 256, 256) || upload_raw(h, &L.co, m.o, 256, 256);
     };
@@ -433,7 +446,7 @@ extern "C" int etude_create(int device, const float* weights_host, size_t n_floa
     }
     RawLinear on_t = take_linear(bl, 1, 256), off_t = take_linear(bl, 1, 256), mpe_t = take_linear(bl, 1, 256), vel_t = take_linear(bl, 128, 256);
     if (!rc && bl.pos != n_floats) rc = fail("etude_create: weight layout consumed %zu of %zu floats", bl.pos, n_floats);
-    if (!rc) guard(upload_linear(h, &h->kv_all, kvw, kvb, 1536, 256));
+    if (!rc) guard(upload_linear(h, &h->kv_hm, kvw, kvb, 1536, 256) || upload_linear(h, &h->kv2, kv2w, kv2b, 512, 256));
     if (!rc) guard(upload_heads(h, &h->heads_f, on_f, off_f, mpe_f, vel_f) || upload_heads(h, &h->heads_t, on_t, off_t, mpe_t, vel_t));
     if (!rc) {
         // decoder.pos_embedding_freq followed by a copy of its first 32 rows: the LN epilogue's 32-row residual boxes start
@@ -534,6 +547,7 @@ static int set_func_attrs_once() {
     set_smem((const void*)attention2_kernel<96>, kAttn2SmemBytes);
     set_smem((const void*)attention4_kernel<128>, kAttn4SmemBytes);
     set_smem((const void*)attention4_kernel<96>, kAttn4SmemBytes);
+    set_smem((const void*)cross_attn_kernel, kCrossAttnSmemBytes);
 #ifdef ETUDE_HAVE_ATTN_QKV_CTA1
     set_smem((const void*)attn_qkv_kernel, kAttnQkvSmemBytes);
 #endif
@@ -684,6 +698,36 @@ static int launch_attention(const void* q, int64_t q_rows, int q_ld, int q_col0,
     {
         char what[96];
         snprintf(what, sizeof what, "attention gen%d n_seq=%d Lq=%d Lk=%d", gen, n_seq, Lq, Lk);
+        if (debug_sync(what, st)) return -1;
+    }
+    return 0;
+}
+
+// Decoder cross-attention with its K|V projection fused in (cross_attn.cuh): x bf16 [n_frames * 256, 256] (the encoder
+// output), w_hm bf16 [512, 256] / bias_hm [512] one layer's head-major [Wk_h; Wv_h], q bf16 [q_rows, 256] with frame f's
+// 88 queries at row f * q_seq_stride (0: one table for every frame) -> context bf16 [n_frames * 88, 256].
+static int launch_cross_attn(const void* x, const __nv_bfloat16* w_hm, const float* bias_hm, const void* q, int64_t q_rows, int q_seq_stride,
+                             int n_frames, __nv_bfloat16* out, cudaStream_t st, Profile* prof) {
+    if (n_frames < 1) return fail("cross_attn: n_frames=%d", n_frames);
+    if (q_seq_stride != 0 && q_seq_stride != kNotes) return fail("cross_attn: q_seq_stride=%d (88 or 0)", q_seq_stride);
+    if (q_rows < 1 || (int64_t)(n_frames - 1) * q_seq_stride + kNotes > q_rows)
+        return fail("cross_attn: %lld query rows do not cover %d frames", (long long)q_rows, n_frames);
+    CUtensorMap tx, tw, tq;
+    if (make_tmap(&tx, x, (uint64_t)n_frames * 256, 256, 256, 256)) return -1;
+    if (make_tmap_ex(&tw, w_hm, 512, 256, 256, 128, 32, 2)) return -1;
+    if (make_tmap(&tq, q, (uint64_t)q_rows, 256, 256, 128)) return -1;
+    CrossAttnParams p{};
+    p.n_frames = n_frames; p.q_seq_stride = q_seq_stride; p.bias = bias_hm; p.out = out;
+    p.scale_log2e = 1.4426950408889634f / 8.0f;
+    const int grid = std::min(n_frames, num_sms_cached());
+    const double fl = 2.0 * n_frames * 256.0 * 512.0 * 256.0 + 4.0 * n_frames * kHeads * (double)kNotes * 256.0 * kHeadDim;
+    cudaEvent_t ev = prof ? prof->begin(PC_ATTN_FUSED, st, fl, 0.0) : nullptr;
+    cross_attn_kernel<<<grid, kXaThreads, kCrossAttnSmemBytes, st>>>(tx, tw, tq, p);
+    if (prof) prof->end(ev, st);
+    CUDA_OK(cudaGetLastError());
+    {
+        char what[64];
+        snprintf(what, sizeof what, "cross_attn n_frames=%d", n_frames);
         if (debug_sync(what, st)) return -1;
     }
     return 0;
@@ -864,6 +908,14 @@ extern "C" int etude_k_gemm(const void* a, const void* w, const float* bias, int
     return fail("etude_k_gemm: only the bias epilogue with K == 256 and N %% 256 == 0 is built into the product library "
                 "(epilogue %d, N=%d, K=%d needs libetude_b200_dev.so)", epilogue, N, K);
 #endif
+}
+
+extern "C" int etude_k_cross_attn(const void* x, const void* w_hm, const float* bias_hm, const void* q, int64_t q_rows, int q_seq_stride,
+                                  int n_frames, void* out, void* stream) {
+    if (!x || !w_hm || !bias_hm || !q || !out) return fail("etude_k_cross_attn: null argument");
+    if (set_func_attrs_once()) return -1;
+    return launch_cross_attn(x, (const __nv_bfloat16*)w_hm, bias_hm, q, q_rows, q_seq_stride, n_frames, (__nv_bfloat16*)out, (cudaStream_t)stream,
+                             nullptr);
 }
 
 extern "C" int etude_k_attention(const void* q, int64_t q_rows, int q_ld, int q_col0, int q_seq_stride, const void* kv, int kv_ld,
@@ -1148,7 +1200,7 @@ extern "C" int etude_logmel(etude_handle_t* h, const float* wave, const int64_t*
 
 // ------------------------------------------------------------------------------------------------ model forward
 struct Workspace {  // every activation is bf16 [tokens, width]; nothing fp32 between kernels
-    __nv_bfloat16* x; __nv_bfloat16* qkv; __nv_bfloat16* ctx; __nv_bfloat16* kv;
+    __nv_bfloat16* x; __nv_bfloat16* ctx; __nv_bfloat16* kv;
     __nv_bfloat16* d; __nv_bfloat16* dqkv; __nv_bfloat16* dctx; __nv_bfloat16* dq; __nv_bfloat16* t;
 };
 static size_t carve(Workspace* ws, uint8_t* base, int nw, int frames) {
@@ -1157,9 +1209,8 @@ static size_t carve(Workspace* ws, uint8_t* base, int nw, int frames) {
     auto take = [&](size_t bytes) { uint8_t* p = base ? base + off : nullptr; off += (bytes + 1023) & ~size_t(1023); return p; };
     Workspace w;
     w.x = (__nv_bfloat16*)take(NT * 256 * 2);
-    w.qkv = (__nv_bfloat16*)take(NT * 768 * 2);
     w.ctx = (__nv_bfloat16*)take(NT * 256 * 2);
-    w.kv = (__nv_bfloat16*)take(NT * 1536 * 2);
+    w.kv = (__nv_bfloat16*)take(NT * 512 * 2);   // layer 2's K|V for the attention-probabilities output only
     w.d = (__nv_bfloat16*)take(ND * 256 * 2);
     w.dqkv = (__nv_bfloat16*)take(ND * 768 * 2);
     w.dctx = (__nv_bfloat16*)take(ND * 256 * 2);
@@ -1305,9 +1356,12 @@ static int forward_impl(etude_handle_t* h, const ForwardIO& io, int nw, void* wo
     }
     if (!io.rolls_A && !io.rolls_B) return 0;   // encode only
     // --- decoder, frequency -> note (Decoder_SPEC2MIDI.forward part 1, amt_apc.py:159-183)
-    if (gemm_bias(ws.x, h->kv_all, NT, ws.kv, st, prof)) return -1;  // K|V of all three cross-attentions
+    // Cross-attentions: K|V projected inside the attention kernel, per frame, never stored (cross_attn.cuh).
+    auto cross = [&](int l, const __nv_bfloat16* q, int64_t q_rows, int q_stride) -> int {
+        return launch_cross_attn(ws.x, h->kv_hm.w + (size_t)l * 512 * 256, h->kv_hm.b + l * 512, q, q_rows, q_stride, NF, ws.dctx, st, prof);
+    };
     // layer zero: cross-attention with the input-independent queries, then fc_o + LN + FFN + LN (residual = the query embedding)
-    if (launch_attention(h->q0, 128, 256, 0, 0, ws.kv, 1536, 0, 256, NF, kNotes, kBins, ws.dctx, nullptr, st, prof)) return -1;
+    if (cross(0, h->q0, 128, 0)) return -1;
     if (launch_chain(ws.dctx, h->dec0.co, &h->dec0.f1, &h->dec0.f2, h->dec0.ln_g, h->dec0.ln_b, h->pos_freq_bf16, kNotes, 3 * kNotes, ws.d, ND,
                      st, prof)) return -1;
     for (int l = 0; l < 2; ++l) {
@@ -1316,8 +1370,12 @@ static int forward_impl(etude_handle_t* h, const ForwardIO& io, int nw, void* wo
         if (launch_attention(ws.dqkv, ND, 768, 0, kNotes, ws.dqkv, 768, 256, 512, NF, kNotes, kNotes, ws.dctx, nullptr, st, prof)) return -1;
         if (launch_chain(ws.dctx, L.o, nullptr, nullptr, L.ln_g, L.ln_b, ws.d, 0, ND, ws.d, ND, st, prof)) return -1;
         if (gemm_bias(ws.d, L.cq, ND, ws.dq, st, prof)) return -1;
-        if (launch_attention(ws.dq, ND, 256, 0, kNotes, ws.kv, 1536, (l + 1) * 512, (l + 1) * 512 + 256, NF, kNotes, kBins, ws.dctx,
-                             (l == 1) ? io.attention : nullptr, st, prof)) return -1;
+        if (l == 1 && io.attention) {   // the 9-tuple's attention probabilities: attention2 on a stored K|V of layer 2
+            if (gemm_bias(ws.x, h->kv2, NT, ws.kv, st, prof)) return -1;
+            if (launch_attention(ws.dq, ND, 256, 0, kNotes, ws.kv, 512, 0, 256, NF, kNotes, kBins, ws.dctx, io.attention, st, prof)) return -1;
+        } else if (cross(l + 1, ws.dq, ND, kNotes)) {
+            return -1;
+        }
         if (launch_chain(ws.dctx, L.co, &L.f1, &L.f2, L.ln_g, L.ln_b, ws.d, 0, ND, ws.d, ND, st, prof)) return -1;
     }
     auto heads = [&](const Linear& W, const __nv_bfloat16* src, void* const* rolls, float* logits, int time_major) -> int {

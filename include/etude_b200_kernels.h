@@ -32,6 +32,15 @@ int etude_k_attention(const void* q_dev, int64_t q_rows, int q_ld, int q_col0, i
                       int kv_ld, int k_col0, int v_col0, int n_seq, int Lq, int Lk, void* out_bf16_dev, float* probs_dev,
                       void* stream);
 
+/* Cross-attention of a frequency-axis decoder layer with its K|V projection fused in (reference amt_apc.py:342-368): frames
+ * of 256 encoder tokens, 88 queries, 4 heads x 64:  out[f*88 + i, 64h..] = softmax(Q_h(f) K_h^T / 8) V_h  with
+ * K_h | V_h = x_f [Wk_h; Wv_h]^T + bias.  x_dev: bf16 [n_frames * 256, 256].  w_hm_dev: bf16 [512, 256] HEAD-MAJOR -- row
+ * h*128 + r holds Wk row 64h + r (r < 64) or Wv row 64h + r - 64; bias_hm_dev fp32 [512] likewise.  q_dev: bf16 [q_rows, 256]
+ * with frame f's queries at rows f*q_seq_stride.. (q_seq_stride 88, or 0: one table for every frame).  out_dev: bf16
+ * [n_frames * 88, 256]. */
+int etude_k_cross_attn(const void* x_dev, const void* w_hm_dev, const float* bias_hm_dev, const void* q_dev, int64_t q_rows,
+                       int q_seq_stride, int n_frames, void* out_dev, void* stream);
+
 /* Self-attention of an encoder layer with the Q|K|V projection fused in (reference amt_apc.py:342-368), sequences of 256
  * tokens, 4 heads x 64:  out[s*256 + i, 64h..] = softmax((x Wq_h^T + bq_h)(x Wk_h^T + bk_h)^T / 8) (x Wv_h^T + bv_h).
  * x_dev / out_dev: bf16 [n_seq * 256, 256].  w_hm_dev: bf16 [768, 256] HEAD-MAJOR -- row h*192 + r holds fc_q row 64h + r
